@@ -6,12 +6,21 @@ through the B200 hot path, with the CPU reference timed beside it.
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference [--steps K --warmup W]              # the reference's algorithm on host cores
     python bench.py --sweep                                              # BASELINE config 5 (needs ≥2 ranks)
+    python bench.py --dump-outputs DIR ...                               # also save the last timed step's outputs
 
 One JSON line on stdout (rank 0).  `value` = whole-job images/s with the batch already resident in HBM;
 `e2e` = the same through `Trainer.step_from_host` (pinned host batch → H2D → iteration → loss D2H);
 `roofline` = the dominant hand-written kernel (SyncBN backward) replayed on the model's 84 layer shapes and
 timed with CUDA events on the launching stream; `cpu_baseline` = the oracle restatement of the reference loop
-on the host cores (bounded sample).  Nothing here reads /root/reference.
+on the host cores (bounded sample).  Nothing here reads the reference project.
+
+`--dump-outputs DIR` writes what the last of the `--steps` timed iterations returned to rank 0 as float32 arrays:
+DIR/loss.npy (the rank-mean loss), DIR/loss_items.npy (the fused loss kernel's 8 report scalars: bce, cel, total,
+Σp, Σt, Σp·t, unreduced bce sum, n; absent for `--impl torch`) and DIR/logits.npy (N×1×H×W, at most 16×1×384×384 =
+9.4 MB).  The inputs and the initial weights are seeded, so two builds run with the same arguments can be compared
+output for output.  Two runs of one build with the same arguments compute the same arrays: cuDNN picks its algorithms
+by heuristics here rather than by timing them, since algorithms that round differently make two runs of the training
+loop drift apart step by step.
 """
 from __future__ import annotations
 
@@ -50,7 +59,17 @@ def parse():
                     help="BASELINE config 4: one size of {256,320,384} per batch (rank-shared RNG), as the reference's multi-scale collate")
     ap.add_argument("--no-parity-check", action="store_true", help="skip the untimed world>1 parity leg")
     ap.add_argument("--no-extras", action="store_true", help="skip the ride-along measurements (multi-scale, sweep, stock-torch arm)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy (float32)")
     return ap.parse_args()
+
+
+def dump_outputs(out_dir: str, outputs) -> None:
+    """`--dump-outputs`: the (loss, loss items, logits) that `forward_backward_update` returned, as float32 .npy files"""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in zip(("loss", "loss_items", "logits"), outputs):
+        if isinstance(t, torch.Tensor):
+            np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().float().cpu().numpy())
 
 
 def peaks():
@@ -657,9 +676,9 @@ def run_b200_arm(args):
 
     dtype = torch.bfloat16 if args.dtype == "bf16" else torch.float32
     args.warmup = max(3, args.warmup)          # timing rule: at least 3 warm-up iterations
-    torch.backends.cudnn.benchmark = True
-    if os.environ.get("SOD_CUDNN_BENCH_LIMIT"):      # experiment knob: 0 = let cuDNN's autotuner try every engine (default 10)
-        torch.backends.cudnn.benchmark_limit = int(os.environ["SOD_CUDNN_BENCH_LIMIT"])
+    # cuDNN's heuristics, not its autotuner: the autotuner times candidate algorithms afresh in every process and may
+    # pick different ones, so two runs on the same inputs would round differently and drift apart as training proceeds
+    torch.backends.cudnn.benchmark = False
     log('building trainer')
     if args.impl == "torch":
         tr = TorchEagerTrainer(args.model, dtype)
@@ -674,7 +693,7 @@ def run_b200_arm(args):
         import random as _random
         sizes = (256, 320, 384)
         rng = _random.Random(0)
-        order = [0, 1, 2] + [rng.randrange(3) for _ in range(4096)]
+        order = [0, 1, 2] + [rng.randrange(3) for _ in range(args.warmup + args.steps)]
         host = [synth_batch(1234 + rank + 100 * i, BS, sizes[k]) for k in range(3) for i in range(nb)]
         seen = [0, 0, 0]
         pick = []
@@ -684,7 +703,7 @@ def run_b200_arm(args):
         mean_pixels = sum(sizes[k] ** 2 for k in order[:args.warmup + args.steps][args.warmup:]) / max(args.steps, 1)
     else:
         host = [synth_batch(1234 + rank + 100 * i, BS, SIZE) for i in range(nb)]
-        pick = [i % nb for i in range(8192)]
+        pick = [i % nb for i in range(args.warmup + args.steps)]
         mean_pixels = SIZE * SIZE
     host = [(x.pin_memory(), m.pin_memory()) for x, m in host]
     dev = [(x.cuda(non_blocking=True), m.cuda(non_blocking=True)) for x, m in host]
@@ -731,12 +750,20 @@ def run_b200_arm(args):
     rid = torch.cuda.nvtx.range_start("timed")      # start/end range: process-wide (backward runs on autograd's thread)
     clk.mark()
     w0 = args.warmup
-    ms = timed(lambda i: tr.forward_backward_update(*dev[pick[w0 + i]]), args.steps)
+    last = {}
+
+    def timed_step(i):
+        last["out"] = tr.forward_backward_update(*dev[pick[w0 + i]])
+    ms = timed(timed_step, args.steps)
     clk.mark()
     torch.cuda.nvtx.range_end(rid)
     clk.__exit__()
     launches = _lib.launches - l0
     log(f'timed region done: {ms / args.steps:.2f} ms/step')
+    if args.dump_outputs:           # before the end-to-end arm replays the graph and overwrites its output buffers
+        if rank == 0:
+            dump_outputs(args.dump_outputs, last["out"])
+        sync_all()
     value = world * BS * args.steps / (ms * 1e-3)
 
     # -- end-to-end arm: pinned host batch in, loss out, every step ------------------------------------

@@ -1,8 +1,12 @@
-"""bench.py's reference arm runs on CPU: check the JSON-line contract the driver parses (keys, units, types)."""
+"""bench.py's output contract: the JSON line (keys, units, types) on the reference arm, which runs on CPU, and the arrays
+`--dump-outputs` writes on the GPU arm."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -38,3 +42,16 @@ def test_reference_arm_world2_is_the_gloo_ddp_syncbn_loop():
     d = json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][0])
     assert d["n_gpus"] == 2 and "2 gloo ranks" in d["cpu_baseline"]["sample"] and "2 CPU ranks" in d["config"]["workload"]
     assert d["value"] > 0 and d["e2e"]["value"] == d["value"]
+
+
+@pytest.mark.gpu
+def test_dump_outputs_writes_the_last_timed_step(tmp_path):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "3", "--no-extras",
+                          "--no-cpu-baseline", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    d = json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][0])
+    assert d["steps"] == 2
+    loss, items, logits = (np.load(tmp_path / f"{n}.npy") for n in ("loss", "loss_items", "logits"))
+    assert loss.dtype == items.dtype == logits.dtype == np.float32
+    assert loss.shape == () and items.shape == (8,) and logits.shape == (16, 1, 320, 320)
+    assert loss == items[2] and items[7] == logits.size and np.isfinite(logits).all()

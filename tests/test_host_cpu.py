@@ -66,29 +66,29 @@ def test_model_plugin_contract():
     assert network.cp_res50.recompute and not network.res50.recompute
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference only exists in the build container")
-def test_model_plugin_is_bit_identical_to_reference():
-    import subprocess, sys
-    code = r'''
-import sys, types, torch, hashlib
-sys.path.insert(0, "/root/reference"); sys.path.insert(0, %r)
-m = types.ModuleType("torchvision.models.utils"); m.load_state_dict_from_url = lambda *a, **k: {}
-sys.modules["torchvision.models.utils"] = m
-for n in ("openpyxl", "thop"):
-    mm = types.ModuleType(n); mm.load_workbook = mm.Workbook = mm.profile = None; sys.modules[n] = mm
-import torch.utils.model_zoo as mz; mz.load_url = lambda *a, **k: {}
-from utils.misc import init_seed
-import network as ref
-from distributed_sod_project_b200 import network as mine
-init_seed(0); a = ref.res50(); init_seed(0); b = mine.res50()
-assert list(a.state_dict()) == list(b.state_dict())
-assert all(torch.equal(x, y) for x, y in zip(a.state_dict().values(), b.state_dict().values()))
-x = torch.randn(2, 3, 64, 64)
-assert torch.equal(a(x), b(x))
-print("IDENTICAL")
-''' % ROOT
-    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True)
-    assert "IDENTICAL" in out.stdout, out.stderr[-2000:]
+def test_model_plugin_is_bit_identical_to_reference(golden):
+    """res50 after `init_seed(0)` against the reference's res50 (tests/golden/model_res50_init.npz, tools/make_golden.py):
+    the same state_dict keys in the same order and bit-identical initial values (sha256 of every entry), and the same
+    output on one seeded input.  The outputs are held to a tolerance, not to the bit: the CPU convolutions' summation
+    order depends on the thread count and instruction set of the host that computes them (1 vs 8 threads moves the
+    eval-mode output by 2e-6 and the train-mode output, whose deepest BN normalises 8 samples, by 1.1e-4 of its range)."""
+    import sys
+    sys.path.insert(0, os.path.join(ROOT, "tools"))
+    from make_golden import tensor_digest
+    from distributed_sod_project_b200 import network
+    from distributed_sod_project_b200.utils import init_seed
+    g = golden("model_res50_init.npz")
+    init_seed(0)
+    m = network.res50()
+    sd = m.state_dict()
+    assert list(sd) == list(g["names"])
+    for name, want in zip(sd, g["digests"]):
+        assert tensor_digest(sd[name]) == want, name
+    x = torch.from_numpy(g["x"])
+    with torch.no_grad():
+        for mode, tol in (("eval", 1e-5), ("train", 1e-3)):
+            got, want = getattr(m, mode)()(x).numpy(), g[f"out_{mode}"]
+            assert np.abs(got - want).max() <= tol * np.abs(want).max(), mode
 
 
 def test_flat_params_layout_cpu():

@@ -18,6 +18,7 @@ the DDP gradient mean == gradient of mean_r(loss_r).  (Parity unpinned for apex 
 """
 from __future__ import annotations
 
+import hashlib
 import os
 import sys
 import types
@@ -188,6 +189,30 @@ def step_vectors(model_name: str, world: int, bs: int, size: int, iters: int, ta
     np.savez_compressed(os.path.join(OUT, f"step_{tag}.npz"), **out)
 
 
+def tensor_digest(t: torch.Tensor) -> str:
+    """sha256 over dtype, shape and the raw bytes of a tensor: equal digests == bit-identical tensors"""
+    t = t.detach().contiguous()
+    return hashlib.sha256(f"{t.dtype}{tuple(t.shape)}".encode() + t.numpy().tobytes()).hexdigest()
+
+
+def model_vectors():
+    """the reference res50 right after `init_seed(0)`: a digest of every state_dict entry (the full state is 100 MB) and
+    its output on one seeded input, in eval mode and then in train mode"""
+    import network
+    from utils.misc import init_seed
+    init_seed(0)
+    model = network.res50()
+    sd = model.state_dict()
+    names, digests = list(sd), [tensor_digest(v) for v in sd.values()]      # before a train-mode forward moves the BN buffers
+    x = torch.randn(2, 3, 64, 64, generator=torch.Generator().manual_seed(0))
+    with torch.no_grad():
+        out_eval = model.eval()(x)
+        out_train = model.train()(x)
+    np.savez_compressed(os.path.join(OUT, "model_res50_init.npz"), names=np.array(names), digests=np.array(digests),
+                        x=x.numpy(), out_eval=out_eval.numpy(), out_train=out_train.numpy())
+    print("model_res50_init:", len(names), "state_dict entries")
+
+
 def main():
     os.makedirs(OUT, exist_ok=True)
     install_reference()
@@ -196,6 +221,10 @@ def main():
         step_vectors("res50", 1, 4, 320, 3, "res50_w1_s320", keep_logits=(0, 1), logits_stride=2)
         step_vectors("res50", 1, 16, 320, 2, "res50_w1_s320_bs16", keep_logits=(0, 1), logits_stride=4)
         return
+    if "--only-model" in sys.argv:
+        model_vectors()
+        return
+    model_vectors()
     loss_kats()
     sgd_kats()
     # 64x64 / bs 2 leaves 8 samples under the deepest BN: a deliberately ill-conditioned edge case (kept for the
